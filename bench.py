@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — claim allocations/sec on the BASELINE.json workload.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one Allocate batch: 10,000 mixed 1g/2g/3g/7g MIG claims (generation order, NOT node-sorted)
 over 125 nodes x 8 GPUs, evaluated against the freshly loaded inventory (BASELINE.md cfg2 = configs[1]).
@@ -62,6 +62,17 @@ def config(world: int, aligned: bool = False) -> dict:
             "inventory": "fresh per step (DRA_F_FRESH_INVENTORY)"}
 
 
+def dump_outputs(d: str, out: np.ndarray, inv: np.ndarray | None = None) -> None:
+    """What a caller of the timed call receives, one float64 array per record field (every field is an integer of at
+    most 32 bits, so the values are exact): out_<field>.npy for the OutRecs, inventory_<field>.npy for the live
+    inventory the call leaves behind (N = 1 only; at N > 1 a rank's inventory is authoritative for its own nodes)."""
+    os.makedirs(d, exist_ok=True)
+    for prefix, rec in (("out", out), ("inventory", inv)):
+        if rec is not None:
+            for f in rec.dtype.names:
+                np.save(os.path.join(d, f"{prefix}_{f}.npy"), rec[f].astype(np.float64))
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -113,8 +124,9 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
-def cpu_oracle_rate(w_list, threads: int, budget_s: float):
-    """allocations/s of the CPU oracle on the concatenated workload; returns (rate, reps, seconds)."""
+def cpu_oracle_rate(w_list, threads: int, steps: int, warmup: int):
+    """allocations/s of the CPU oracle on the concatenated workload: `warmup` untimed batches, then `steps` timed ones;
+    returns (rate, steps, seconds, OutRecs, inventory) with the outputs of the last timed batch."""
     from oracle import oracle as O
     O.build()
     pkg = importlib.import_module("k8s-dra-driver_b200")
@@ -136,18 +148,16 @@ def cpu_oracle_rate(w_list, threads: int, budget_s: float):
     scratch = gpus.copy()
     p = lambda a: a.ctypes.data  # noqa: E731
     times = []
-    t_end = time.perf_counter() + budget_s
-    reps = 0
-    while reps < 5 or (time.perf_counter() < t_end and reps < 20000):
+    for i in range(warmup + steps):
         scratch[:] = gpus                                   # fresh inventory per step, as on the GPU
         t0 = time.perf_counter()
         rc = lib.dra_oracle_allocate_mt(p(scratch), len(scratch), p(node_off), len(node_off) - 1, p(table),
                                         p(claims), len(claims), None, p(out), len(out), threads)
-        times.append(time.perf_counter() - t0)
+        if i >= warmup:
+            times.append(time.perf_counter() - t0)
         assert rc == 0
-        reps += 1
     med = statistics.median(times)
-    return len(claims) / med, reps, sum(times)
+    return len(claims) / med, len(times), sum(times), out, scratch
 
 
 def thread_candidates(cores: int, n_node: int):
@@ -156,36 +166,40 @@ def thread_candidates(cores: int, n_node: int):
     return sorted({1, top} | {t for t in (8, 16, 32, 64) if t < top})
 
 
-def best_cpu_rate(w_list, cores: int, n_node: int, budget_s: float):
-    """(rate, threads, reps, seconds, {threads: rate}) of the fastest thread count."""
+def best_cpu_rate(w_list, cores: int, n_node: int, steps: int, warmup: int):
+    """(rate, threads, reps, seconds, {threads: rate}, OutRecs, inventory) of the fastest thread count; the outputs are
+    those of its last timed batch."""
     per, best = {}, None
     for th in thread_candidates(cores, n_node):
-        rate, reps, secs = cpu_oracle_rate(w_list, th, budget_s)
+        rate, reps, secs, out, inv = cpu_oracle_rate(w_list, th, steps, warmup)
         per[th] = rate
         if best is None or rate > best[0]:
-            best = (rate, th, reps, secs)
-    return (*best, per)
+            best = (rate, th, reps, secs, out, inv)
+    return (*best[:4], per, *best[4:])
 
 
-def cpu_arm(pkg, w, cores: int, budget_s: float) -> dict:
+def cpu_arm(pkg, w, cores: int, steps: int, warmup: int):
     """The CPU arm on one global workload: the oracle port (the checker, plain restatement of the spec) and, beside
     it, the tuned port of the same spec (oracle/dra_oracle_tuned.c: no allocation in the call, parallel bucketing,
-    -O3 -march=native, shift/AND fit map) — both with every thread count in by_threads, the best one reported."""
-    rate, th, reps, secs, per = best_cpu_rate([w], cores, w.n_node, budget_s)
-    d = {"value": rate, "unit": UNIT, "cores": th, "kind": "port",
-         "sample": f"{reps} full batches of {w.n_claim} claims, median; CPU oracle of spec/ALLOCATION.md (plain restatement, the "
+    -O3 -march=native, shift/AND fit map) — both with every thread count in by_threads, the best one reported, each
+    thread count timed over `steps` batches after `warmup` untimed ones.  Returns (result dict, OutRecs, inventory),
+    the outputs of the oracle port's last timed batch at its best thread count."""
+    rate, th, reps, secs, per, out, inv = best_cpu_rate([w], cores, w.n_node, steps, warmup)
+    d = {"value": rate, "unit": UNIT, "cores": th, "kind": "port", "timed_steps": reps, "warmup": warmup,
+         "sample": f"{reps} timed full batches of {w.n_claim} claims after {warmup} untimed, median; CPU oracle of spec/ALLOCATION.md (plain restatement, the "
                    f"parity checker), nodes spread over a persistent thread pool; best of the thread counts in by_threads "
                    f"(the reference's Go allocator is absent from the snapshot and Go is not installed)",
          "value_1_thread": per[1], "by_threads": {str(k): v for k, v in per.items()}, "host_cores": cores}
     try:
         from oracle import tuned as T
-        tr, tth, tper = T.best_rate(w, cores, budget_s)
+        tr, tth, tper = T.best_rate(w, cores, steps, warmup)
         d["port_tuned"] = {"value": tr, "unit": UNIT, "cores": tth, "kind": "port-tuned", "by_threads": {str(k): v for k, v in tper.items()},
+                           "timed_steps": steps, "warmup": warmup,
                            "note": "same spec, same bytes out (checked against the oracle before timing); a reported baseline, "
                                    "what a CPU implementation written for speed concedes"}
     except Exception as e:                                  # the tuned port is optional test infrastructure
         d["port_tuned"] = {"unavailable": str(e)[:200]}
-    return d
+    return d, out, inv
 
 
 def run_reference(args):
@@ -198,8 +212,9 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     from oracle import oracle as O
     O.build()
-    budget = max(1.5, min(20.0, 0.005 * (args.steps + args.warmup)))
-    cpu = cpu_arm(pkg, w, cores, budget)
+    cpu, out, inv = cpu_arm(pkg, w, cores, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, inv if world == 1 else None)
     rate = cpu["value"]
     n = w.n_claim
     line = {"impl": "reference", "metric": METRIC, "value": rate, "unit": UNIT, "n_gpus": world,
@@ -320,14 +335,15 @@ def run_ours(args):
         if args.steps * ms_per_step < 250:                     # a short run: keep the sampler up long enough for > 1 sample
             time.sleep(0.25)
     ctx.sync()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, result(w, d_out), ctx.get_inventory() if world == 1 else None)
     launches = (ctx.launch_count() - launches0) * args.steps // (args.steps + max(3, args.warmup))
     value = n_claim / (ms_per_step * 1e-3)
 
     # ---- per-kernel device times (separate pass: event pairs around every kernel) --------------------
     ctx.set_profiling(True)
     stage = {}
-    reps = min(50, max(10, args.steps))
-    for _ in range(reps):
+    for _ in range(args.steps):
         if world > 1:
             dist.barrier()                         # (the gather waits for its peers: without this a rank's host-side delay would be timed)
         flush.fill_(1); step_dev(); ctx.sync()
@@ -430,7 +446,7 @@ def run_ours(args):
                 "us_per_batch": ms_per_step * 1e3}
         line.update(extras)
         if world == 1:
-            line["cpu_baseline"] = cpu_arm(pkg, w, cores, 1.5)
+            line["cpu_baseline"] = cpu_arm(pkg, w, cores, args.steps, args.warmup)[0]
         print(json.dumps(line))
     pin_c.free(); pin_o.free()
     ctx.close()
@@ -441,10 +457,10 @@ def run_ours(args):
 
 def run_extras(pkg, O, ctx, timer, torch, dev, world, rank, load, make_step, result, args) -> dict:
     """Every other BASELINE config, the sharded configs[2] and a size where sharding should pay, UnsuitableNodes and the
-    pod mode — same timing discipline as the headline (events, L2 flush, max over ranks), fewer steps, parity against
+    pod mode — same timing discipline as the headline (events, L2 flush, max over ranks, --steps timed steps), parity against
     the oracle before each timing.  Keys are added to the one JSON line."""
     R, S = pkg.records, pkg.synth
-    steps = max(10, min(40, args.steps))
+    steps = args.steps
     F = pkg.api.F_FRESH_INVENTORY
     out = {}
 
@@ -494,7 +510,7 @@ def run_extras(pkg, O, ctx, timer, torch, dev, world, rank, load, make_step, res
             ref = O.unsuitable(inv, w.node_off, w.table, claims[:500], pod_off[:501], cn, co, flags=ofl)
             assert bits[: len(ref) - 1].tobytes() == ref[: len(ref) - 1].tobytes()
             ts = []
-            for _ in range(12):
+            for _ in range(args.steps):
                 t0 = time.perf_counter(); ctx.unsuitable(claims, pod_off, flags=fl); ts.append(time.perf_counter() - t0)
             ctx.set_profiling(True); ctx.unsuitable(claims, pod_off, flags=fl)
             k_us = list(ctx.timings_us().values())[0]
@@ -508,9 +524,9 @@ def run_extras(pkg, O, ctx, timer, torch, dev, world, rank, load, make_step, res
         po = ppo[: sub + 1]; pc = pw.claims[: po[-1]]
         ctx.set_table(pw.table); ctx.set_inventory(pw.gpus, pw.node_off)
         ff = np.unpackbits(ctx.unsuitable(pc, po), bitorder="little")[: sub * 64]
-        def med(fn, n=5):                                   # (the first call of a shape also grows buffers: median of the later ones)
+        def med(fn):                                        # (the first call of a shape also grows buffers: median of the later ones)
             r = fn(); ts = []
-            for _ in range(n):
+            for _ in range(args.steps):
                 t0 = time.perf_counter(); r = fn(); ts.append(time.perf_counter() - t0)
             return r, statistics.median(ts)
         exb, t_ex = med(lambda: ctx.unsuitable(pc, po, flags=pkg.api.F_EXHAUSTIVE))
@@ -523,7 +539,7 @@ def run_extras(pkg, O, ctx, timer, torch, dev, world, rank, load, make_step, res
                            "pairs": sub * 64, "suitable_first_fit": int(ff.sum()), "suitable_exhaustive": int(ex.sum()),
                            "flipped_to_suitable": int((ex & ~ff).sum()), "unsuitable_exhaustive_e2e_ms": t_ex * 1e3,
                            "allocate_pods_exhaustive_e2e_ms": t_ap * 1e3, "allocate_pods_first_fit_e2e_ms": t_ap_ff * 1e3,
-                           "note": "host wall clock of the C-ABI call, median of 5 after a first call; 64 nodes = 64 sequential chains of ~312 pods: "
+                           "note": f"host wall clock of the C-ABI call, median of {args.steps} after a first call; 64 nodes = 64 sequential chains of ~312 pods: "
                                    "the exhaustive call is bound by the longest chain of searches, not by the GPU's width", "pods": 20_000, "claims": int(pw.n_claim),
                            "search_limit_slots": int((po_out["status"] == R.ST_SEARCH_LIMIT).sum()), "parity": "bit-exact vs oracle"}
     return out
@@ -532,7 +548,8 @@ def run_extras(pkg, O, ctx, timer, torch, dev, world, rank, load, make_step, res
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps of every timed loop: the headline, the e2e leg, the per-kernel "
+                    "stage pass, the other configs, UnsuitableNodes, pod mode and, per thread count, the CPU ports")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-direct", action="store_true", help="e2e leg: copy-engine transfers around the kernel instead of direct host I/O")
@@ -542,7 +559,11 @@ def main():
     ap.add_argument("--e2e-copy", action="store_true", help="N > 1, e2e leg: H2D copy of the global claim array in front of the call instead of zero-copy ingest")
     ap.add_argument("--align", action="store_true", help="N > 1: device-side rendezvous of the ranks (dra_peer_rendezvous_device) between the untimed L2 "
                     "flush and the timed step; measured at N = 2: no difference (29.46 vs 29.48 us), off by default")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                    "(float64; the inputs are seeded, so runs with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

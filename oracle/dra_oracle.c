@@ -380,6 +380,7 @@ static void run_nodes(const mt_arg* a)
 static struct {
     pthread_t* th; int n;                       /* workers (the caller works too) */
     _Atomic uint64_t gen;                       /* batch generation */
+    uint64_t start_gen;                         /* gen when the current workers were created */
     _Atomic uint32_t next, done;                /* next node to take; workers finished with this generation */
     const mt_arg* job;
     _Atomic int stop, sleepers;
@@ -399,7 +400,7 @@ static void take_nodes(const mt_arg* a)
 static void* pool_worker(void* unused)
 {
     (void)unused;
-    uint64_t seen = 0;
+    uint64_t seen = pool.start_gen;             /* batches before this worker existed are not its business */
     for (;;) {
         uint32_t spins = 0;
         while (atomic_load_explicit(&pool.gen, memory_order_acquire) == seen && !atomic_load(&pool.stop)) {
@@ -447,6 +448,7 @@ static int pool_resize(int workers)
     if (!pool.th) return -1;
     static int at_exit_set;
     if (!at_exit_set) { atexit(pool_shutdown); pthread_atfork(NULL, NULL, pool_after_fork_child); at_exit_set = 1; }
+    pool.start_gen = atomic_load(&pool.gen);
     for (int t = 0; t < workers; t++)
         if (pthread_create(&pool.th[t], NULL, pool_worker, NULL)) { pool.n = t; pool_shutdown(); return -1; }
     pool.n = workers;

@@ -48,8 +48,9 @@ def allocate(gpus, node_off, table, claims, out_off=None, n_out=None, threads: i
     return out[:n_out], g
 
 
-def rate(w, threads: int, budget_s: float):
-    """allocations/s (median over full batches, fresh inventory per batch, like the GPU's timed step)."""
+def rate(w, threads: int, steps: int, warmup: int):
+    """allocations/s (median over `steps` full batches after `warmup` untimed ones, fresh inventory per batch, like the
+    GPU's timed step)."""
     L = lib()
     gpus, claims = w.gpus.copy(), np.ascontiguousarray(w.claims)
     scratch = gpus.copy()
@@ -57,24 +58,24 @@ def rate(w, threads: int, budget_s: float):
     off, t = np.ascontiguousarray(w.node_off, dtype=np.uint32), np.ascontiguousarray(w.table)
     oo = None if w.out_off is None else np.ascontiguousarray(w.out_off, dtype=np.uint32)
     p = lambda a: None if a is None else a.ctypes.data  # noqa: E731
-    ts, reps, t_end = [], 0, time.perf_counter() + budget_s
-    while reps < 5 or (time.perf_counter() < t_end and reps < 20000):
+    ts = []
+    for i in range(warmup + steps):
         scratch[:] = gpus
         t0 = time.perf_counter()
         rc = L.dra_oracle_tuned_allocate(p(scratch), len(scratch), p(off), len(off) - 1, p(t), p(claims), len(claims), p(oo), p(out), w.n_out, threads)
-        ts.append(time.perf_counter() - t0)
+        if i >= warmup:
+            ts.append(time.perf_counter() - t0)
         assert rc == 0
-        reps += 1
     return len(claims) / statistics.median(ts), out[: w.n_out].copy(), scratch.copy()
 
 
-def best_rate(w, cores: int, budget_s: float):
+def best_rate(w, cores: int, steps: int, warmup: int):
     """(best rate, its thread count, {threads: rate}); the result is compared with the plain oracle first."""
     ref, ref_inv = O.allocate(w.gpus, w.node_off, w.table, w.claims, w.out_off, w.n_out)
     per, best = {}, None
     top = max(1, min(cores, w.n_node))
     for th in sorted({1, top} | {x for x in (4, 8, 16, 32, 64) if x < top}):
-        r, out, inv = rate(w, th, budget_s / 2)
+        r, out, inv = rate(w, th, steps, warmup)
         if out.tobytes() != ref.tobytes() or inv.tobytes() != ref_inv.tobytes():
             raise RuntimeError("tuned CPU port differs from the oracle")
         per[th] = r

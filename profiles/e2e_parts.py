@@ -1,5 +1,5 @@
 import importlib, os, sys, time, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 pkg = importlib.import_module("k8s-dra-driver_b200")
 R=pkg.records
 w = pkg.synth.cfg2()

@@ -1,5 +1,5 @@
 import importlib, os, sys, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 pkg = importlib.import_module("k8s-dra-driver_b200")
 s = torch.cuda.Stream(); torch.cuda.set_stream(s)
 ctx = pkg.api.Context(device=0, stream=s.cuda_stream)

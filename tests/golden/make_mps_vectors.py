@@ -1,20 +1,22 @@
 """Extracts the reference's own MPS-limit test table into tests/golden/mps_limits.json.
 
-Source: /root/reference/api/nvidia.com/resource/gpu/v1alpha1/sharing_test.go:37-149
-(TestMpsPerDevicePinnedMemoryLimitNormalize, 14 table cases).  Run in the build container only
-(/root/reference does not exist on the GPU box); the JSON is what travels.
+Source: api/nvidia.com/resource/gpu/v1alpha1/sharing_test.go:37-149 of NVIDIA/k8s-dra-driver
+(TestMpsPerDevicePinnedMemoryLimitNormalize, 14 table cases).  The tests read only the JSON, so they need no
+checkout of that project:
+
+  python tests/golden/make_mps_vectors.py <k8s-dra-driver checkout>
 """
 import json
 import os
 import re
 import sys
 
-SRC = "/root/reference/api/nvidia.com/resource/gpu/v1alpha1/sharing_test.go"
+SRC = os.path.join("api", "nvidia.com", "resource", "gpu", "v1alpha1", "sharing_test.go")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "mps_limits.json")
 
 
-def main():
-    text = open(SRC).read()
+def main(reference_root):
+    text = open(os.path.join(reference_root, SRC)).read()
     body = text[text.index("testCases := []struct"):text.index("for _, tc := range testCases")]
     body = body[body.index("}{") + 2:]
     cases = []
@@ -39,4 +41,4 @@ def main():
 
 
 if __name__ == "__main__":
-    sys.exit(main())
+    sys.exit(main(sys.argv[1]))

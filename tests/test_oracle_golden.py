@@ -136,8 +136,9 @@ def test_oracle_matches_naive_on_homogeneous_nodes(pkg, oracle, seed, model, wid
 def test_oracle_mt_equals_single_thread(pkg, oracle):
     w = pkg.synth.cfg2(5000, 60)
     a, ga = oracle.allocate(w.gpus, w.node_off, w.table, w.claims)
-    b, gb = oracle.allocate(w.gpus, w.node_off, w.table, w.claims, threads=5)
-    assert a.tobytes() == b.tobytes() and ga.tobytes() == gb.tobytes()
+    for threads in (5, 2, 8, 3):              # each change of thread count restarts the worker pool after earlier batches
+        b, gb = oracle.allocate(w.gpus, w.node_off, w.table, w.claims, threads=threads)
+        assert a.tobytes() == b.tobytes() and ga.tobytes() == gb.tobytes(), threads
 
 
 # ---- frozen golden files (drift check) ----
